@@ -2,6 +2,7 @@
 """bench.py -- headline benchmark of the nufhe_b200 engine (contract: see the task statement).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--gate nand|mux] [--impl reference]
+                    [--dump-outputs DIR]
 
 One "step" = one bootstrapped gate (default gate_nand) over a batch of B ciphertexts per GPU on synthetic data:
 seeded keys in the reference's RNG order, uniformly random LWE samples as operands (the bootstrap does the same work
@@ -58,7 +59,15 @@ def parse_args():
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-extras', action='store_true', help='skip the mux / ntt / sweep legs (headline line only)')
     ap.add_argument('--ntt-transforms', type=int, default=262144)
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write the ciphertexts the last one returned (a, b, current_variances; '
+                         'rank 0 under torchrun) as DIR/<name>.npy')
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be at least 1 and --warmup at least 0')
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs writes the outputs of the GPU path (--impl b200)')
+    return args
 
 
 def host_cores():
@@ -144,6 +153,28 @@ def c0_committed():
     except Exception:
         return {'available': False, 'why': 'the reference closures need /root/reference (build container only); '
                                            'run tools/c0_baseline.py there'}
+
+
+DUMP_LIMIT_BYTES = 64 * 10**6
+
+
+def dump_outputs(directory, a, b, current_variances):
+    """Write one step's destination ciphertexts (host arrays) as DIR/<name>.npy.  The int32 torus values go out as
+    float64, which holds every one exactly.  When all ciphertexts would exceed DUMP_LIMIT_BYTES, a fixed seeded
+    sample of them is written instead, with their indices in rows.npy."""
+    import numpy
+    n = b.shape[0]
+    per_ct = 8 * a.shape[-1] + 8 + 4 + 8          # a, b, current_variances and the index of a sampled ciphertext
+    arrays = {'a': a.astype(numpy.float64), 'b': b.astype(numpy.float64),
+              'current_variances': current_variances.astype(numpy.float32)}
+    if n * per_ct > DUMP_LIMIT_BYTES:
+        keep = (DUMP_LIMIT_BYTES - 4096) // per_ct    # 4096: room for the .npy headers
+        rows = numpy.sort(numpy.random.RandomState(SEED).choice(n, keep, replace=False))
+        arrays = {k: v[rows] for k, v in arrays.items()}
+        arrays['rows'] = rows.astype(numpy.float64)
+    os.makedirs(directory, exist_ok=True)
+    for name, arr in arrays.items():
+        numpy.save(os.path.join(directory, name + '.npy'), arr)
 
 
 def metric_name(args):
@@ -369,6 +400,11 @@ def run_b200_arm(args):
     ms_total = timed(main['device_step'], args.steps)
     sampler.stop_flag.set()
     sampler.join(timeout=2)
+    if args.dump_outputs and rank == 0:
+        # now: the stand-alone key switch timed below writes into the same buffers
+        dest = main['dest']
+        dump_outputs(args.dump_outputs, dest.a.cpu().numpy(), dest.b.cpu().numpy(),
+                     dest.current_variances.cpu().numpy())
     for _ in range(max(1, args.warmup // 2)):
         main['e2e_step']()
     ms_e2e = timed(main['e2e_step'], args.steps)

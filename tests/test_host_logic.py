@@ -306,6 +306,34 @@ def test_uint_bit_helpers_roundtrip():
     assert (bitarray_to_uintarray(uintarray_to_bitarray(ys)) == ys).all()
 
 
+def test_bench_dump_outputs_exact_and_bounded(tmp_path):
+    """bench.py --dump-outputs: every int32 survives the float64 file exactly; above the size limit a seeded sample
+    of whole ciphertexts is written, the same one every time, and the files stay within the limit."""
+    import bench
+    rng = numpy.random.RandomState(3)
+
+    def case(n):
+        return (rng.randint(-2**31, 2**31, (n, 500), dtype=numpy.int32), rng.randint(-2**31, 2**31, n, dtype=numpy.int32),
+                rng.uniform(0, 1e-3, n).astype(numpy.float32))
+
+    a, b, cv = case(64)
+    bench.dump_outputs(str(tmp_path / 'small'), a, b, cv)
+    got = {k: numpy.load(str(tmp_path / 'small' / (k + '.npy'))) for k in ('a', 'b', 'current_variances')}
+    assert got['a'].dtype == numpy.float64 and (got['a'] == a).all() and (got['b'] == b).all()
+    assert got['current_variances'].dtype == numpy.float32 and (got['current_variances'] == cv).all()
+    assert not (tmp_path / 'small' / 'rows.npy').exists()
+
+    a, b, cv = case(20000)                      # 20000 x 4020 bytes > 64 MB
+    for d in ('big1', 'big2'):
+        bench.dump_outputs(str(tmp_path / d), a, b, cv)
+    assert sum(f.stat().st_size for f in (tmp_path / 'big1').iterdir()) <= bench.DUMP_LIMIT_BYTES
+    rows = numpy.load(str(tmp_path / 'big1' / 'rows.npy')).astype(numpy.int64)
+    assert (numpy.diff(rows) > 0).all() and len(rows) > 15000
+    assert (rows == numpy.load(str(tmp_path / 'big2' / 'rows.npy'))).all()
+    assert (numpy.load(str(tmp_path / 'big1' / 'a.npy')) == a[rows]).all()
+    assert (numpy.load(str(tmp_path / 'big1' / 'b.npy')) == b[rows]).all()
+
+
 def test_pickle_wire_compatibility_with_reference_parameter_classes():
     """The parameter objects nufhe pickles into every dump: ours carry the same attributes and, with
     compat.use_reference_pickle_paths(), the same class paths; a pickle made by the REFERENCE's classes
