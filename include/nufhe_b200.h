@@ -69,7 +69,9 @@ int nb_ff_elementwise(nb_ctx *ctx, int op, const uint64_t *a, const uint64_t *b,
 
 /* ---- bootstrap key: BootstrapKey / TransformedTGswSampleArray (bootstrap.py:44-92, tgsw.py:99-130).
  * Re-lays `rows` reference rows (each 2*2*2*1024 uint64) into the engine's internal row format:
- * nb_bk_row_u64() uint64 per row (the 8 planes re-ordered and un-Montgomery-ed + 2 correction planes). */
+ * nb_bk_row_u64() uint64 per row: the NTT part (the 8 planes re-ordered and un-Montgomery-ed + 2 correction planes,
+ * 10 x 1024) and the FFT part (the 16 float64 limb spectra of the row, 16384).  bk_int holds all `rows` NTT parts first,
+ * then all FFT parts; the gate entry points with LWE dimension n read a key of exactly n rows. */
 size_t nb_bk_row_u64(void);
 int nb_bk_prepare(nb_ctx *ctx, const uint64_t *bk_ref, uint64_t *bk_int, size_t rows);
 

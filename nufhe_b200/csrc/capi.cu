@@ -3,9 +3,11 @@
 #include <cstdlib>
 #include <cstring>
 #include <string>
+#include <type_traits>
 #include <nvtx3/nvToolsExt.h>
 #include "../../include/nufhe_b200.h"
 #include "kernels.cuh"
+#include "fft_kernels.cuh"
 #include "tables.h"
 
 using namespace nb;
@@ -29,6 +31,8 @@ struct nb_ctx {
     size_t cv_words;
     int force_chunks;                    // developer knob: chunk count of every multi-wave launch (0 = automatic)
     int stagger_cycles;                  // start-up offset of the second CTA per SM in single-wave launches
+    int use_fft;                         // gate bootstraps above wide_max take the FP64 FFT kernel (fft_kernels.cuh)
+    FftTables *d_fft_tab;                // its twiddle tables (br_fft.cuh)
     std::string err;
 };
 
@@ -91,6 +95,7 @@ int nb_ctx_create(int device, void *stream, nb_ctx **out)
     ctx->d_ph_fwd = ctx->d_ph_inv = ctx->d_ones512 = nullptr;
     ctx->d_sched = nullptr; ctx->d_state = nullptr; ctx->sched_words = ctx->state_words = 0;
     ctx->d_cv_blocks = nullptr; ctx->cv_words = 0;
+    ctx->d_fft_tab = nullptr;
     *out = ctx;   // returned even on failure so that nb_last_error() can be read; caller destroys it
     NB_ON_DEVICE(ctx);
     cudaDeviceProp prop;
@@ -104,6 +109,8 @@ int nb_ctx_create(int device, void *stream, nb_ctx **out)
         ctx->force_chunks = e ? atoi(e) : 0;
         e = getenv("NUFHE_B200_STAGGER");
         ctx->stagger_cycles = e ? atoi(e) : 12000;        // about a quarter of a CMux step (measured best of 0 / 12k / 24k / 36k)
+        e = getenv("NUFHE_B200_FFT");                      // 0: every batch stays on the NTT kernels
+        ctx->use_fft = e ? atoi(e) : 1;
     }
     if (const char *e = getenv("NUFHE_B200_FORCE_RARE_PATH")) {
         // test knob: run the canonicalisation fix-up of the deferred-canonicalisation phases on every task
@@ -122,6 +129,14 @@ int nb_ctx_create(int device, void *stream, nb_ctx **out)
     NB_TRY(check(ctx, cudaMemcpy(ctx->d_ph_inv, pt.inv.data(), NTT_N * sizeof(u64), cudaMemcpyHostToDevice), "memcpy"));
     NB_TRY(check(ctx, cudaMalloc(&ctx->d_ones512, NTT_N * sizeof(u64)), "cudaMalloc"));
     NB_TRY(check(ctx, cudaMemcpy(ctx->d_ones512, pt.ones512.data(), NTT_N * sizeof(u64), cudaMemcpyHostToDevice), "memcpy"));
+    {
+        FftTables ft;
+        make_fft_tables(ft);
+        NB_TRY(check(ctx, cudaMalloc(&ctx->d_fft_tab, sizeof(FftTables)), "cudaMalloc"));
+        NB_TRY(check(ctx, cudaMemcpy(ctx->d_fft_tab, &ft, sizeof(FftTables), cudaMemcpyHostToDevice), "memcpy"));
+    }
+    NB_TRY(check(ctx, cudaFuncSetAttribute(blind_rotate_fft_kernel<BrFft>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                           (int)br_fft_smem_bytes<BrFft>()), "cudaFuncSetAttribute(blind_rotate fft)"));
     NB_TRY(check(ctx, cudaFuncSetAttribute(blind_rotate_kernel<BrDefault>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                            (int)br_smem_bytes<BrDefault>()), "cudaFuncSetAttribute(blind_rotate)"));
     NB_TRY(check(ctx, cudaFuncSetAttribute(blind_rotate_kernel<BrWide>, cudaFuncAttributeMaxDynamicSharedMemorySize,
@@ -189,6 +204,7 @@ void nb_ctx_destroy(nb_ctx *ctx)
     if (ctx->d_sched) cudaFree(ctx->d_sched);
     if (ctx->d_state) cudaFree(ctx->d_state);
     if (ctx->d_cv_blocks) cudaFree(ctx->d_cv_blocks);
+    if (ctx->d_fft_tab) cudaFree(ctx->d_fft_tab);
     delete ctx;
 }
 
@@ -291,7 +307,9 @@ int nb_ff_elementwise(nb_ctx *ctx, int op, const uint64_t *a, const uint64_t *b,
     return launch_check(ctx, "ff_elementwise_kernel");
 }
 
-size_t nb_bk_row_u64(void) { return BK_ROW_U64; }
+// per key row: the NTT planes (BK_ROW_U64) and the FFT spectra (FFT_ROW_U64).  A key of `rows` rows is laid out as
+// all NTT rows first, then all spectra rows (the FFT kernel finds them after n NTT rows).
+size_t nb_bk_row_u64(void) { return BK_ROW_U64 + FFT_ROW_U64; }
 
 int nb_bk_prepare(nb_ctx *ctx, const uint64_t *bk_ref, uint64_t *bk_int, size_t rows)
 {
@@ -302,7 +320,21 @@ int nb_bk_prepare(nb_ctx *ctx, const uint64_t *bk_ref, uint64_t *bk_int, size_t 
     size_t total = rows * NTT_N, blocks = (total + 255) / 256, cap = (size_t)ctx->sm_count * 16;
     bk_prepare_kernel<<<(int)(blocks < cap ? blocks : cap), 256, 0, ctx->stream>>>((const u64 *)bk_ref, (u64 *)bk_int,
                                                                                   ctx->d_ones512, rows);
-    return launch_check(ctx, "bk_prepare_kernel");
+    NB_TRY(launch_check(ctx, "bk_prepare_kernel"));
+    // the key spectra of the FFT kernel: exact int32 coefficients by the inverse transform of the reference key, split
+    // into two 16-bit limbs, folded, twisted, transformed and scaled by 1/512 (br_fft.cuh)
+    const size_t polys = rows * 8;
+    u64 *plain = nullptr;
+    i32 *coef = nullptr;
+    NB_TRY(check(ctx, cudaMallocAsync((void **)&plain, polys * NTT_N * sizeof(u64), ctx->stream), "cudaMallocAsync"));
+    NB_TRY(check(ctx, cudaMallocAsync((void **)&coef, polys * NTT_N * sizeof(i32), ctx->stream), "cudaMallocAsync"));
+    blocks = (polys * NTT_N + 255) / 256;
+    bk_plain_kernel<<<(int)(blocks < cap ? blocks : cap), 256, 0, ctx->stream>>>((const u64 *)bk_ref, plain, polys * NTT_N);
+    ntt_inverse_kernel<true><<<ntt_grid(ctx, polys), NTT_SWEEP_THREADS, ntt_smem_bytes(NTT_RAW_U64_BYTES), ctx->stream>>>(plain, coef, ctx->d_ph_inv, polys);
+    fft_key_kernel<<<(unsigned)(polys * 2), 64, 0, ctx->stream>>>(coef, reinterpret_cast<cplx *>((u64 *)bk_int + rows * BK_ROW_U64), ctx->d_fft_tab);
+    NB_TRY(launch_check(ctx, "fft_key_kernel"));
+    NB_TRY(check(ctx, cudaFreeAsync(plain, ctx->stream), "cudaFreeAsync"));
+    return check(ctx, cudaFreeAsync(coef, ctx->stream), "cudaFreeAsync");
 }
 
 }  // extern "C"
@@ -360,7 +392,10 @@ template <class Cfg> static int launch_br_cfg(nb_ctx *ctx, BlindRotateArgs &p)
         p.sched = ctx->d_sched; p.state = ctx->d_state;
         grid = slots;
     }
-    blind_rotate_kernel<Cfg><<<(int)grid, Cfg::THREADS, br_smem_bytes<Cfg>(), ctx->stream>>>(p, ctx->d_ph_fwd, ctx->d_ph_inv);
+    if constexpr (std::is_same_v<Cfg, BrFft>)
+        blind_rotate_fft_kernel<Cfg><<<(int)grid, Cfg::THREADS, br_fft_smem_bytes<Cfg>(), ctx->stream>>>(p, ctx->d_fft_tab);
+    else
+        blind_rotate_kernel<Cfg><<<(int)grid, Cfg::THREADS, br_smem_bytes<Cfg>(), ctx->stream>>>(p, ctx->d_ph_fwd, ctx->d_ph_inv);
     return NB_OK;
 }
 
@@ -377,6 +412,8 @@ static int launch_br(nb_ctx *ctx, BlindRotateArgs &p)
     }
     if (p.batch <= ctx->wide2_max) return launch_br_cfg<BrWide2>(ctx, p);
     if (p.batch <= ctx->wide_max) return launch_br_cfg<BrWide>(ctx, p);
+    // gate bootstraps (the key handle then has exactly n rows, so the spectra follow the n NTT rows)
+    if (ctx->use_fft && !p.plain && !p.bara && p.n > 0) return launch_br_cfg<BrFft>(ctx, p);
     return launch_br_cfg<BrDefault>(ctx, p);
 }
 

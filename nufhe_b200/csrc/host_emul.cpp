@@ -238,3 +238,72 @@ void emul_ff_sub(const u64 *a, const u64 *b, u64 *out, size_t n)
 { for (size_t i = 0; i < n; i++) out[i] = ff_sub(a[i], b[i]); }
 
 }  // extern "C"
+
+// ---- the FFT external product (br_fft.cuh) ----------------------------------------------------------------------
+// the two limb spectra of every key polynomial of `rows` reference rows (2,2,2,1024 Montgomery NTT values each), in the
+// layout the kernels read: rows x [m][limb][512] complex = rows x FFT_ROW_U64 doubles' bits (kernels.cuh:
+// fft_key_kernel computes the same on the device)
+static void fft_key_row(const u64 *bk_ref_row, const FftTables &T, cplx *out)
+{
+    std::vector<u64> plain(NTT_N);
+    std::vector<i32> k(NTT_N);
+    std::vector<cplx> f(FFT_STRIDE);
+    for (int m = 0; m < 8; m++) {
+        for (int x = 0; x < NTT_N; x++) plain[x] = ff_mul(ff_canon(bk_ref_row[m * NTT_N + x]), FF_RINV);
+        emul_ntt_inverse_i32(plain.data(), k.data(), 1);
+        for (int limb = 0; limb < 2; limb++) {
+            for (int t = 0; t < 64; t++) fft_key_phase1(t, k.data(), limb, f.data(), T);
+            for (int t = 0; t < 64; t++) fft_fwd2(t, f.data(), T);
+            for (int t = 0; t < 64; t++) fft_key_phase3_store(t, f.data(), out + (m * 2 + limb) * FFT_M);
+        }
+    }
+}
+
+static const FftTables &fft_tables()
+{
+    static FftTables T;
+    static bool init = false;
+    if (!init) { make_fft_tables(T); init = true; }
+    return T;
+}
+
+extern "C" {
+
+void emul_fft_key_spectra(const u64 *bk_ref, u64 *out, size_t rows)
+{
+    for (size_t r = 0; r < rows; r++)
+        fft_key_row(bk_ref + r * 8 * NTT_N, fft_tables(), reinterpret_cast<cplx *>(out + r * FFT_ROW_U64));
+}
+
+// One CMux step (rot != NULL) or plain external product (rot == NULL: acc <- key (x) acc) of the FFT kernel for `nct`
+// ciphertexts (acc: nct x 2 x 1024), phase by phase as the kernel runs them.  *err_max: the largest distance to the
+// nearest integer seen before rounding, over all output coefficients.
+void emul_fft_step(i32 *acc, const u64 *bk_ref_row, const int *rot, int nct, double *err_max)
+{
+    const FftTables &T = fft_tables();
+    std::vector<cplx> key(FFT_KEY_SPECTRA * FFT_M);
+    fft_key_row(bk_ref_row, T, key.data());
+    std::vector<cplx> w((size_t)nct * 4 * FFT_STRIDE);
+    *err_max = 0;
+    for (int c = 0; c < nct; c++)
+        for (int mi = 0; mi < 2; mi++)
+            for (int t = 0; t < 64; t++) {
+                cplx *f2 = w.data() + (c * 4 + mi * 2) * FFT_STRIDE;
+                if (rot) fft_step_fwd1<true>(t, acc + (c * 2 + mi) * NTT_N, f2, T, rot[c]);
+                else fft_step_fwd1<false>(t, acc + (c * 2 + mi) * NTT_N, f2, T, 0);
+            }
+    for (int s = 0; s < nct * 4; s++) for (int t = 0; t < 64; t++) fft_fwd2(t, w.data() + s * FFT_STRIDE, T);
+    for (int s = 0; s < nct * 4; s++) for (int t = 0; t < 64; t++) fft_fwd3(t, w.data() + s * FFT_STRIDE);
+    for (int i = 0; i < FFT_M; i++) fft_step_mac(i, w.data(), 4 * FFT_STRIDE, nct, key.data());
+    for (int s = 0; s < nct * 4; s++) for (int t = 0; t < 64; t++) fft_inv3(t, w.data() + s * FFT_STRIDE, T);
+    for (int s = 0; s < nct * 4; s++) for (int t = 0; t < 64; t++) fft_inv2(t, w.data() + s * FFT_STRIDE, T);
+    for (int c = 0; c < nct; c++)
+        for (int mo = 0; mo < 2; mo++)
+            for (int t = 0; t < 64; t++) {
+                const cplx *f2 = w.data() + (c * 4 + mo * 2) * FFT_STRIDE;
+                if (rot) fft_step_inv1<true>(t, acc + (c * 2 + mo) * NTT_N, f2, T, err_max);
+                else fft_step_inv1<false>(t, acc + (c * 2 + mo) * NTT_N, f2, T, err_max);
+            }
+}
+
+}  // extern "C"

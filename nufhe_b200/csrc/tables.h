@@ -6,6 +6,8 @@
 #include <vector>
 #include "ntt_lane.cuh"
 #include "br_phases.cuh"
+#include "br_fft.cuh"
+#include <cmath>
 
 namespace nb {
 
@@ -39,5 +41,18 @@ struct PhaseTables {
             }
     }
 };
+
+// Twiddles of the FFT external product (br_fft.cuh), each component computed in long double and rounded once to
+// double: |error| <= 2^-53 per component (the bound in DESIGN.md section 8 uses this).
+inline void make_fft_tables(FftTables &T)
+{
+    const long double pi = 3.141592653589793238462643383279502884L;
+    auto w = [&](int m) { m &= FFT_M - 1; return cplx{(double)cosl(2 * pi * m / FFT_M), (double)sinl(2 * pi * m / FFT_M)}; };
+    for (int m = 0; m < FFT_M; m++) {
+        T.tw1[m] = w((m & 63) * (m >> 6));
+        T.twist[m] = cplx{(double)cosl(pi * m / NTT_N), (double)sinl(pi * m / NTT_N)};
+    }
+    for (int m = 0; m < 64; m++) T.tw2[m] = w(8 * (m >> 3) * (m & 7));
+}
 
 }  // namespace nb
