@@ -16,13 +16,22 @@
 // X^1024 + 1; the inverse runs the conjugate DFT, which returns 512 z: the factor 1/512 lives in the key spectra.
 //
 // The 512-point DFT is 8 x 8 x 8, j = 64 j0 + 8 j1 + j2, k = k0 + 8 k1 + 64 k2:
-//     pass 1 (task t = 8 j1 + j2):  DFT8 over j0 -> k0, times W^(t k0)              (W = exp(2 pi i / 512))
+//     pass 1 (task t = 8 j1 + j2):  DFT8 over j0 -> k0, times W^(t k0)              (W = exp(2 pi i / 512) = omega^4)
 //     pass 2 (task t = 8 k0 + j2):  DFT8 over j1 -> k1, times W^(8 j2 k1)
 //     pass 3 (task t = 8 k0 + k1):  DFT8 over j2 -> k2
 // every pass in place: element (a, b, c) lives at index 64 a + 8 b + c, so the spectrum X[k0 + 8 k1 + 64 k2] ends at
 // index 64 k0 + 8 k1 + k2.  The MAC is point-wise, so it never needs natural order; the key spectra are stored in the
-// same order.  The inverse runs the mirror image (conjugate DFT8 first, then the conjugate twiddle; passes 3, 2, 1) and
-// ends in natural order.  Index i is stored at i + i / 8: every warp access of the three passes is bank-conflict free.
+// same order.  The inverse runs the mirror image (passes 3, 2, 1, each the conjugate DFT8 after the conjugate twiddle)
+// and ends in natural order.  Index i is stored at i + i / 8: every warp access of the three passes is bank-conflict
+// free.
+//
+// Pass 1 merges the twist into its twiddle.  With twist omega^(64 j0 + t) = omega^t e^(i pi j0 / 16),
+//     W^(t k0) DFT8_k0(a'_(64 j0 + t) omega^(64 j0 + t)) = omega^(t (1 + 4 k0)) DFT8_k0(a'_(64 j0 + t) e^(i pi j0 / 16)),
+// so a task multiplies its inputs by 8 compile-time constants e^(i pi j0 / 16) (j0 = 0 is free, j0 = 4 is a rot8) and
+// its outputs by 8 entries of one per-thread table, tw[64 k0 + t] = omega^(t (1 + 4 k0)), which it loads once for both
+// of its polynomials.  The inverse pass 1 does the conjugate: the conjugate twiddle that pass 2 of the inverse would
+// apply to its outputs (same element, same thread) and the untwist's omega^(-t) are conj(tw) on its inputs, the
+// conjugate constants on its outputs.
 //
 // Every function is __host__ __device__ and every floating-point operation is explicit (fma() where fused, __dadd_rn /
 // __dmul_rn on the device, which nvcc never contracts; the host emulator is built with -ffp-contract=off), so the host
@@ -41,6 +50,14 @@ constexpr int FFT_ROW_U64 = FFT_KEY_SPECTRA * FFT_M * 2;     // 16384 u64 = 128 
 constexpr double FFT_ROUND_MAGIC = 6755399441055744.0;      // 1.5 * 2^52
 constexpr double FFT_DIGIT_BIAS = 4503599627370496.0 + 512.0; // 2^52 + 512
 constexpr double FFT_SQRT1_2 = 0.70710678118654752440;
+// cos(pi j0 / 16), 0 <= j0 <= 8 (sin(pi j0 / 16) = cos(pi (8 - j0) / 16)), each rounded once: the factors
+// e^(i pi j0 / 16) of pass 1 (j0 = 0 and 4 are not multiplied by: identity and rot8)
+NB_HDC double fft_cos16(int j)
+{
+    return j == 0 ? 1.0 : j == 1 ? 0.9807852804032304491262 : j == 2 ? 0.9238795325112867561282
+         : j == 3 ? 0.8314696123025452370788 : j == 4 ? 0.7071067811865475244008 : j == 5 ? 0.5555702330196022247428
+         : j == 6 ? 0.3826834323650897717285 : j == 7 ? 0.1950903220161282678483 : 0.0;
+}
 
 NB_HD int fft_pos(int i) { return i + (i >> 3); }
 
@@ -133,17 +150,26 @@ NB_HD cplx ld_c_global(const cplx *p)
 #endif
 }
 
+// by e^(s i pi / 4) = (1 + s i) / sqrt 2, s = +1 (INV = false) or -1
+template <bool INV> NB_HD cplx c_rot8(cplx a)
+{
+    return INV ? cplx{d_mul(d_add(a.re, a.im), FFT_SQRT1_2), d_mul(d_sub(a.im, a.re), FFT_SQRT1_2)}
+               : cplx{d_mul(d_sub(a.re, a.im), FFT_SQRT1_2), d_mul(d_add(a.re, a.im), FFT_SQRT1_2)};
+}
+// by e^(s i pi j0 / 16), 0 < j0 < 8 (a compile-time constant wherever the caller's loop is unrolled)
+template <bool INV> NB_HD cplx c_rot16(cplx a, int j0)
+{
+    if (j0 == 4) return c_rot8<INV>(a);
+    return c_mul(a, cplx{fft_cos16(j0), INV ? -fft_cos16(8 - j0) : fft_cos16(8 - j0)});
+}
+
 // 8-point DFT in place, natural order in and out: y_k = sum_j x_j e^(s 2 pi i jk / 8), s = +1 (INV = false) or -1.
 // Radix 2, decimation in frequency; the only non-trivial constants are e^(+-i pi / 4) = (1 +- i) / sqrt 2.
 template <bool INV> NB_HD void dft8(cplx *x)
 {
     // by e^(s i pi / 2): s = +1: (a + ib) i = -b + ia; s = -1: b - ia
     auto rot4 = [](cplx a) -> cplx { return INV ? cplx{a.im, -a.re} : cplx{-a.im, a.re}; };
-    // by e^(s i pi / 4) = (1 + s i) / sqrt 2
-    auto rot8 = [](cplx a) -> cplx {
-        return INV ? cplx{d_mul(d_add(a.re, a.im), FFT_SQRT1_2), d_mul(d_sub(a.im, a.re), FFT_SQRT1_2)}
-                   : cplx{d_mul(d_sub(a.re, a.im), FFT_SQRT1_2), d_mul(d_add(a.re, a.im), FFT_SQRT1_2)};
-    };
+    auto rot8 = [](cplx a) -> cplx { return c_rot8<INV>(a); };
     cplx a[4], b[4];
     for (int j = 0; j < 4; j++) { a[j] = c_add(x[j], x[j + 4]); b[j] = c_sub(x[j], x[j + 4]); }
     b[1] = rot8(b[1]); b[2] = rot4(b[2]); b[3] = rot4(rot8(b[3]));
@@ -155,21 +181,27 @@ template <bool INV> NB_HD void dft8(cplx *x)
 }
 
 // ---- tables (host-computed once, read by host emulator and kernels alike) ----------------------------------------
-// tw1[k0 * 64 + t] = W^(t k0) (pass 1), tw2[a * 8 + b] = W^(8 a b) (pass 2, symmetric), twist[j] = omega^j, j < 512;
-// W = e^(2 pi i / 512).  Laid out so that the 32 lanes of a warp read consecutive or identical entries.
+// tw[k0 * 64 + t] = omega^(t (1 + 4 k0)) (pass 1, twist merged in), tw2[a * 8 + b] = W^(8 a b) (pass 2, symmetric);
+// omega = e^(i pi / 1024), W = omega^4.  Laid out so that the 32 lanes of a warp read consecutive or identical entries.
 struct FftTables {
-    cplx tw1[FFT_M];
+    cplx tw[FFT_M];
     cplx tw2[64];
-    cplx twist[FFT_M];
 };
 
-// ---- passes over one polynomial `f` (FFT_STRIDE complex slots) ----------------------------------------------------
-// forward pass 1 from values already in registers: x[j0] = z[64 j0 + t]
-NB_HD void fft_fwd1_store(int t, cplx *x, cplx *f, const FftTables &T)
+// the 8 pass-1 factors of task t, tw[k0] = omega^(t (1 + 4 k0))
+NB_HD void fft_load_tw1(int t, const FftTables &T, cplx *tw)
 {
+    for (int k0 = 0; k0 < 8; k0++) tw[k0] = ld_c(&T.tw[64 * k0 + t]);
+}
+
+// ---- passes over one polynomial `f` (FFT_STRIDE complex slots) ----------------------------------------------------
+// forward pass 1 from values already in registers: x[j0] = a'[64 j0 + t], the folded input before the twist
+// (z[64 j0 + t] = x[j0] omega^(64 j0 + t)); tw from fft_load_tw1
+NB_HD void fft_fwd1_store(int t, cplx *x, cplx *f, const cplx *tw)
+{
+    for (int j0 = 1; j0 < 8; j0++) x[j0] = c_rot16<false>(x[j0], j0);
     dft8<false>(x);
-    st_c(f + fft_pos(t), x[0]);
-    for (int k0 = 1; k0 < 8; k0++) st_c(f + fft_pos(64 * k0 + t), c_mul(x[k0], T.tw1[k0 * 64 + t]));
+    for (int k0 = 0; k0 < 8; k0++) st_c(f + fft_pos(64 * k0 + t), c_mul(x[k0], tw[k0]));
 }
 NB_HD void fft_fwd2(int t, cplx *f, const FftTables &T)
 {
@@ -198,22 +230,22 @@ NB_HD void fft_inv3(int t, cplx *f, const FftTables &T)
     st_c(g, x[0]);
     for (int j2 = 1; j2 < 8; j2++) st_c(g + j2, c_mul(x[j2], c_conj(T.tw2[j2 * 8 + k1])));
 }
-NB_HD void fft_inv2(int t, cplx *f, const FftTables &T)
+// (its output twiddle conj(W^(t' k0)), t' = 8 j1 + j2, is applied by fft_inv1_load)
+NB_HD void fft_inv2(int t, cplx *f)
 {
-    const int base = 64 * (t >> 3) + (t & 7), j2 = t & 7, k0 = t >> 3;
+    const int base = 64 * (t >> 3) + (t & 7);
     cplx x[8];
     for (int k1 = 0; k1 < 8; k1++) x[k1] = ld_c(f + fft_pos(base + 8 * k1));
     dft8<true>(x);
-    for (int j1 = 0; j1 < 8; j1++) {
-        const cplx v = k0 == 0 ? x[j1] : c_mul(x[j1], c_conj(T.tw1[k0 * 64 + 8 * j1 + j2]));
-        st_c(f + fft_pos(base + 8 * j1), v);
-    }
+    for (int j1 = 0; j1 < 8; j1++) st_c(f + fft_pos(base + 8 * j1), x[j1]);
 }
-// inverse pass 1 into registers: x[j0] = 512 z[64 j0 + t] (the 1/512 is in the key spectra)
-NB_HD void fft_inv1_load(int t, const cplx *f, cplx *x)
+// inverse pass 1 into registers, untwisted: x[j0] = 512 a'[64 j0 + t] (the 1/512 is in the key spectra); tw from
+// fft_load_tw1.  conj(tw[k0]) = conj(W^(t k0)) omega^(-t): pass 2's twiddle and the untwist's omega^(-t).
+NB_HD void fft_inv1_load(int t, const cplx *f, const cplx *tw, cplx *x)
 {
-    for (int k0 = 0; k0 < 8; k0++) x[k0] = ld_c(f + fft_pos(64 * k0 + t));
+    for (int k0 = 0; k0 < 8; k0++) x[k0] = c_mul(ld_c(f + fft_pos(64 * k0 + t)), c_conj(tw[k0]));
     dft8<true>(x);
+    for (int j0 = 1; j0 < 8; j0++) x[j0] = c_rot16<true>(x[j0], j0);
 }
 
 // ---- the CMux step ------------------------------------------------------------------------------------------------
@@ -221,7 +253,7 @@ NB_HD void fft_inv1_load(int t, const cplx *f, cplx *x)
 // spectrum of digit polynomial j of ACC[mi]; after it, slot mo * 2 + limb holds output polynomial mo, key limb `limb`.
 
 // forward pass 1 for both digit polynomials of ACC[mi]: task t < 64.  Rotation (X^a - 1) ACC, the unsigned digit
-// u = d + 512 (decomp_udigit), u -> d as 2^52 + u - (2^52 + 512), fold and twist, DFT8, twiddle.
+// u = d + 512 (decomp_udigit), u -> d as 2^52 + u - (2^52 + 512), fold, pass 1 with the twist merged in.
 template <bool ROTATE>
 NB_HD void fft_step_fwd1(int t, const i32 *acc, cplx *f2 /* the 2 digit slots of ACC[mi] */, const FftTables &T, int a)
 {
@@ -233,6 +265,8 @@ NB_HD void fft_step_fwd1(int t, const i32 *acc, cplx *f2 /* the 2 digit slots of
         const i32 c = ROTATE ? rotate_minus_one(acc, idx, ar, flip) : acc[idx];
         tv[h] = (u32)c + (0x80000000u + (1u << 21));
     }
+    cplx tw[8];
+    fft_load_tw1(t, T, tw);
 #if defined(__CUDA_ARCH__)
 #pragma unroll 1
 #endif
@@ -242,9 +276,9 @@ NB_HD void fft_step_fwd1(int t, const i32 *acc, cplx *f2 /* the 2 digit slots of
         for (int j0 = 0; j0 < 8; j0++) {
             const double lo = d_sub(d_from_u32_biased((tv[j0] >> sh) & 1023u), FFT_DIGIT_BIAS);
             const double hi = d_sub(d_from_u32_biased((tv[8 + j0] >> sh) & 1023u), FFT_DIGIT_BIAS);
-            x[j0] = c_mul(cplx{lo, hi}, T.twist[64 * j0 + t]);
+            x[j0] = cplx{lo, hi};
         }
-        fft_fwd1_store(t, x, f2 + j * FFT_STRIDE, T);
+        fft_fwd1_store(t, x, f2 + j * FFT_STRIDE, tw);
     }
 }
 
@@ -268,7 +302,7 @@ NB_HD void fft_step_mac(int i, cplx *w, int stride, int ct, const cplx *key)
     }
 }
 
-// Inverse pass 1 for both limbs of output polynomial mo (task t < 64), untwist, round, recombine, ACC += (or =).
+// Inverse pass 1 for both limbs of output polynomial mo (task t < 64) with the untwist, round, recombine, ACC += (or =).
 // Reports the largest |x - round(x)| through *err_max when it is not null (host emulation only).
 template <bool ACCUMULATE>
 NB_HD void fft_step_inv1(int t, i32 *acc, const cplx *f2 /* slots (mo, limb 0), (mo, limb 1) */, const FftTables &T,
@@ -276,15 +310,17 @@ NB_HD void fft_step_inv1(int t, i32 *acc, const cplx *f2 /* slots (mo, limb 0), 
 {
     u32 r[16];                                          // lo32(c_lo) + (lo32(c_hi) << 16), [j0] and [8 + j0] (+512)
     for (int h = 0; h < 16; h++) r[h] = 0;
+    cplx tw[8];
+    fft_load_tw1(t, T, tw);
 #if defined(__CUDA_ARCH__)
 #pragma unroll 1
 #endif
     for (int limb = 0; limb < 2; limb++) {
         cplx x[8];
-        fft_inv1_load(t, f2 + limb * FFT_STRIDE, x);
+        fft_inv1_load(t, f2 + limb * FFT_STRIDE, tw, x);
         const int sh = 16 * limb;
         for (int j0 = 0; j0 < 8; j0++) {
-            const cplx y = c_mul(x[j0], c_conj(T.twist[64 * j0 + t]));
+            const cplx y = x[j0];
             r[j0] += d_round_lo32(y.re) << sh;
             r[8 + j0] += d_round_lo32(y.im) << sh;
 #if !defined(__CUDA_ARCH__)
@@ -319,9 +355,11 @@ NB_HD void fft_key_phase1(int t, const i32 *k, int limb, cplx *f, const FftTable
             const i32 hi = (i32)(((long long)c - lo) >> 16);     // [-2^15, 2^15]
             v[h] = (double)(limb ? hi : lo);
         }
-        x[j0] = c_mul(cplx{v[0], v[1]}, T.twist[idx]);
+        x[j0] = cplx{v[0], v[1]};
     }
-    fft_fwd1_store(t, x, f, T);
+    cplx tw[8];
+    fft_load_tw1(t, T, tw);
+    fft_fwd1_store(t, x, f, tw);
 }
 NB_HD void fft_key_phase3_store(int t, cplx *f, cplx *out)
 {

@@ -311,6 +311,23 @@ int nb_ff_elementwise(nb_ctx *ctx, int op, const uint64_t *a, const uint64_t *b,
 // all NTT rows first, then all spectra rows (the FFT kernel finds them after n NTT rows).
 size_t nb_bk_row_u64(void) { return BK_ROW_U64 + FFT_ROW_U64; }
 
+#ifdef NB_FFT_PHASE_CLOCKS
+// profiling builds only (tools/fft_phases.py): copy the per-CTA phase clocks of blind_rotate_fft_kernel
+// (fft_kernels.cuh, FFT_CLK_CTAS x FFT_CLK_SLOTS u64) to `out` and, if `reset`, zero them on the device
+int nb_fft_phase_clocks(nb_ctx *ctx, unsigned long long *out, int reset)
+{
+    if (!ctx || !out) return fail(ctx, NB_EINVAL, "nb_fft_phase_clocks: null argument");
+    NB_ON_DEVICE(ctx);
+    NB_TRY(check(ctx, cudaStreamSynchronize(ctx->stream), "cudaStreamSynchronize"));
+    NB_TRY(check(ctx, cudaMemcpyFromSymbol(out, g_fft_phase_clocks, sizeof(g_fft_phase_clocks)), "cudaMemcpyFromSymbol"));
+    if (!reset) return NB_OK;
+    void *d = nullptr;
+    NB_TRY(check(ctx, cudaGetSymbolAddress(&d, g_fft_phase_clocks), "cudaGetSymbolAddress"));
+    NB_TRY(check(ctx, cudaMemset(d, 0, sizeof(g_fft_phase_clocks)), "cudaMemset"));
+    return check(ctx, cudaDeviceSynchronize(), "cudaDeviceSynchronize");
+}
+#endif
+
 int nb_bk_prepare(nb_ctx *ctx, const uint64_t *bk_ref, uint64_t *bk_int, size_t rows)
 {
     if (!ctx || !bk_ref || !bk_int) return fail(ctx, NB_EINVAL, "nb_bk_prepare: null argument");

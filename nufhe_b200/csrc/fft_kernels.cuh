@@ -24,34 +24,76 @@ template <class Cfg> constexpr size_t br_fft_smem_bytes()
     return (size_t)Cfg::CT * 4 * FFT_STRIDE * sizeof(cplx) + sizeof(FftTables) + (size_t)Cfg::CT * 2 * NTT_N * sizeof(i32) + 64;
 }
 
+// Phase clocks (profiling builds only: -DNB_FFT_PHASE_CLOCKS, tools/fft_phases.py).  Thread 0 of each CTA sums the
+// clock64() cycles it spends in each phase of the step (FFT_CLK_FWD1 .. FFT_CLK_INV1), waiting at the step's barriers
+// (FFT_CLK_SYNC) and fetching the next rotation (FFT_CLK_OTHER), and counts the steps; at exit it adds them to
+// g_fft_phase_clocks[blockIdx.x].  The shipped library has none of it: FftClocks is then empty.
+enum { FFT_CLK_FWD1, FFT_CLK_FWD2, FFT_CLK_FWD3, FFT_CLK_MAC, FFT_CLK_INV3, FFT_CLK_INV2, FFT_CLK_INV1, FFT_CLK_SYNC,
+       FFT_CLK_OTHER, FFT_CLK_STEPS, FFT_CLK_SLOTS };
+#ifdef NB_FFT_PHASE_CLOCKS
+constexpr int FFT_CLK_CTAS = 1024;
+__device__ unsigned long long g_fft_phase_clocks[FFT_CLK_CTAS][FFT_CLK_SLOTS];
+__shared__ unsigned long long s_fft_clk[FFT_CLK_SLOTS];     // thread 0's sums (shared memory: no registers held)
+struct FftClocks {
+    long long t = 0;
+    NB_D void start() { t = clock64(); }
+    NB_D void mark(int k) { const long long n = clock64(); if (threadIdx.x == 0) s_fft_clk[k] += n - t; t = n; }
+    NB_D void flush(int tid)
+    {
+        if (tid == 0 && blockIdx.x < FFT_CLK_CTAS)
+            for (int k = 0; k < FFT_CLK_SLOTS; k++) g_fft_phase_clocks[blockIdx.x][k] += s_fft_clk[k];
+    }
+};
+#else
+struct FftClocks {
+    NB_D void start() {}
+    NB_D void mark(int) {}
+    NB_D void flush(int) {}
+};
+#endif
+
 // one CMux step of the CTA's ciphertexts: ACC[ct] += key (x) ((X^rot[ct] - 1) ACC[ct]); key = the row's 16 spectra
-template <class Cfg> NB_D void br_fft_step(cplx *w, const FftTables &T, i32 *acc, const int *rot, const cplx *__restrict__ key, int tid)
+template <class Cfg>
+NB_D void br_fft_step(cplx *w, const FftTables &T, i32 *acc, const int *rot, const cplx *__restrict__ key, int tid, FftClocks &clk)
 {
     constexpr int TH = Cfg::THREADS;
     {   // task (ct * 2 + mi, t): both digit polynomials of ACC[mi]
         const int pm = tid >> 6;
         fft_step_fwd1<true>(tid & 63, acc + pm * NTT_N, w + pm * 2 * FFT_STRIDE, T, rot[pm >> 1]);
     }
+    clk.mark(FFT_CLK_FWD1);
     __syncthreads();
+    clk.mark(FFT_CLK_SYNC);
 #pragma unroll 1
     for (int it = 0; it < 2; it++) { const int task = it * TH + tid; fft_fwd2(task & 63, w + (task >> 6) * FFT_STRIDE, T); }
+    clk.mark(FFT_CLK_FWD2);
     __syncthreads();
+    clk.mark(FFT_CLK_SYNC);
 #pragma unroll 1
     for (int it = 0; it < 2; it++) { const int task = it * TH + tid; fft_fwd3(task & 63, w + (task >> 6) * FFT_STRIDE); }
+    clk.mark(FFT_CLK_FWD3);
     __syncthreads();
+    clk.mark(FFT_CLK_SYNC);
 #pragma unroll 1
     for (int i = tid; i < FFT_M; i += TH) fft_step_mac(i, w, 4 * FFT_STRIDE, Cfg::CT, key);
+    clk.mark(FFT_CLK_MAC);
     __syncthreads();
+    clk.mark(FFT_CLK_SYNC);
 #pragma unroll 1
     for (int it = 0; it < 2; it++) { const int task = it * TH + tid; fft_inv3(task & 63, w + (task >> 6) * FFT_STRIDE, T); }
+    clk.mark(FFT_CLK_INV3);
     __syncthreads();
+    clk.mark(FFT_CLK_SYNC);
 #pragma unroll 1
-    for (int it = 0; it < 2; it++) { const int task = it * TH + tid; fft_inv2(task & 63, w + (task >> 6) * FFT_STRIDE, T); }
+    for (int it = 0; it < 2; it++) { const int task = it * TH + tid; fft_inv2(task & 63, w + (task >> 6) * FFT_STRIDE); }
+    clk.mark(FFT_CLK_INV2);
     __syncthreads();
+    clk.mark(FFT_CLK_SYNC);
     {   // task (ct * 2 + mo, t): both limbs of output polynomial mo
         const int pp = tid >> 6;
         fft_step_inv1<true>(tid & 63, acc + pp * NTT_N, w + pp * 2 * FFT_STRIDE, T);
     }
+    clk.mark(FFT_CLK_INV1);
 }
 
 // Gate bootstraps only (p.bara == null, p.plain == 0): the key handle holds the n NTT rows and, after them, the n rows of
@@ -66,6 +108,10 @@ __global__ void __launch_bounds__(Cfg::THREADS, Cfg::CTAS_PER_SM) blind_rotate_f
     int *rot = reinterpret_cast<int *>(acc + Cfg::CT * 2 * NTT_N);
     __shared__ unsigned s_item, s_entry;
     const int tid = threadIdx.x;
+    FftClocks clk;
+#ifdef NB_FFT_PHASE_CLOCKS
+    if (tid < FFT_CLK_SLOTS) s_fft_clk[tid] = 0;
+#endif
     for (int i = tid; i < (int)(sizeof(FftTables) / 16); i += Cfg::THREADS)
         reinterpret_cast<double2 *>(&T)[i] = reinterpret_cast<const double2 *>(tab_g)[i];
     const cplx *key0 = reinterpret_cast<const cplx *>(p.bk + (size_t)p.n * BK_ROW_U64);
@@ -115,13 +161,19 @@ __global__ void __launch_bounds__(Cfg::THREADS, Cfg::CTAS_PER_SM) blind_rotate_f
         }
         if (tid < Cfg::CT) rot[(step0 & 1) * Cfg::CT + tid] = br2_rotation(p, ct_of(tid), step0);
         __syncthreads();
+        clk.start();
         for (int i = step0; i < step1; i++) {
             int next = 0;
             if (tid < Cfg::CT && i + 1 < step1) next = br2_rotation(p, ct_of(tid), i + 1);
-            br_fft_step<Cfg>(w, T, acc, rot + (i & 1) * Cfg::CT, key0 + (size_t)i * KEY_ROW_CPLX, tid);
+            clk.mark(FFT_CLK_OTHER);
+            br_fft_step<Cfg>(w, T, acc, rot + (i & 1) * Cfg::CT, key0 + (size_t)i * KEY_ROW_CPLX, tid, clk);
             if (tid < Cfg::CT) rot[((i + 1) & 1) * Cfg::CT + tid] = next;
             __syncthreads();
+            clk.mark(FFT_CLK_SYNC);
         }
+#ifdef NB_FFT_PHASE_CLOCKS
+        if (tid == 0) s_fft_clk[FFT_CLK_STEPS] += step1 - step0;
+#endif
 
         if (step1 < p.n) {
             int4 *dst = reinterpret_cast<int4 *>(p.state + (size_t)chain * ACC_WORDS);
@@ -147,6 +199,7 @@ __global__ void __launch_bounds__(Cfg::THREADS, Cfg::CTAS_PER_SM) blind_rotate_f
         }
         if (!p.sched) break;
     }
+    clk.flush(tid);
 }
 
 // ---- key spectra (nb_bk_prepare) ------------------------------------------------------------------------------------

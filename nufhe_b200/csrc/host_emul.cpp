@@ -269,6 +269,14 @@ static const FftTables &fft_tables()
 
 extern "C" {
 
+// the twiddle tables of the FFT kernel: tw (FFT_M complex) then tw2 (64 complex) as interleaved doubles, and the pass-1
+// constants cos(pi j / 16), j = 0..8
+void emul_fft_tables(double *tw, double *cos16)
+{
+    memcpy(tw, &fft_tables(), sizeof(FftTables));
+    for (int j = 0; j <= 8; j++) cos16[j] = fft_cos16(j);
+}
+
 void emul_fft_key_spectra(const u64 *bk_ref, u64 *out, size_t rows)
 {
     for (size_t r = 0; r < rows; r++)
@@ -296,7 +304,7 @@ void emul_fft_step(i32 *acc, const u64 *bk_ref_row, const int *rot, int nct, dou
     for (int s = 0; s < nct * 4; s++) for (int t = 0; t < 64; t++) fft_fwd3(t, w.data() + s * FFT_STRIDE);
     for (int i = 0; i < FFT_M; i++) fft_step_mac(i, w.data(), 4 * FFT_STRIDE, nct, key.data());
     for (int s = 0; s < nct * 4; s++) for (int t = 0; t < 64; t++) fft_inv3(t, w.data() + s * FFT_STRIDE, T);
-    for (int s = 0; s < nct * 4; s++) for (int t = 0; t < 64; t++) fft_inv2(t, w.data() + s * FFT_STRIDE, T);
+    for (int s = 0; s < nct * 4; s++) for (int t = 0; t < 64; t++) fft_inv2(t, w.data() + s * FFT_STRIDE);
     for (int c = 0; c < nct; c++)
         for (int mo = 0; mo < 2; mo++)
             for (int t = 0; t < 64; t++) {

@@ -48,9 +48,9 @@ inline void make_fft_tables(FftTables &T)
 {
     const long double pi = 3.141592653589793238462643383279502884L;
     auto w = [&](int m) { m &= FFT_M - 1; return cplx{(double)cosl(2 * pi * m / FFT_M), (double)sinl(2 * pi * m / FFT_M)}; };
-    for (int m = 0; m < FFT_M; m++) {
-        T.tw1[m] = w((m & 63) * (m >> 6));
-        T.twist[m] = cplx{(double)cosl(pi * m / NTT_N), (double)sinl(pi * m / NTT_N)};
+    for (int m = 0; m < FFT_M; m++) {                  // omega^(t (1 + 4 k0)), t = m & 63, k0 = m >> 6
+        const int e = ((m & 63) * (1 + 4 * (m >> 6))) & (2 * NTT_N - 1);
+        T.tw[m] = cplx{(double)cosl(pi * e / NTT_N), (double)sinl(pi * e / NTT_N)};
     }
     for (int m = 0; m < 64; m++) T.tw2[m] = w(8 * (m >> 3) * (m & 7));
 }

@@ -4,6 +4,12 @@ library (no GPU needed).  The kernel is bound by the integer ALU pipe, so the AL
 the number that predicts its run time; use this to judge an arithmetic change before spending GPU minutes.
 
     python tools/sass_stats.py [--kernel blind_rotate_kernel] [--by-func] [--lib path/to/lib.so]
+    python tools/sass_stats.py --kernel blind_rotate_fft_kernel [--json]
+
+The FP64 FFT kernel (--kernel blind_rotate_fft_kernel, or _ZN2nb23blind_rotate_fft_kernelINS_8BrFftCfgILi4E for the
+4-ciphertext shape) gets its own report: FP64 instructions, the LDS / STS / LDG split and modelled shared-memory / L1
+wavefronts per phase (fft_kernel_stats).  The default stays the NTT kernel: the committed DRAM-traffic capture
+(profiles/r2_traffic.json) carries that kernel's per-phase counts as its fingerprint.
 
 Each SASS instruction is attributed (through nvdisasm's inline chains, the library is built with -lineinfo)
 to the line of `br2_step` in kernels.cuh that called it, i.e. to a phase.  Counts are static: fwd1 / fwd2 /
@@ -76,6 +82,107 @@ def enclosing_functions(path):
     return names
 
 
+FP64 = ('DFMA', 'DADD', 'DMUL')
+FFT_PHASES = ('fwd1', 'fwd2', 'fwd3', 'mac', 'inv3', 'inv2', 'inv1')
+
+
+def block_lines(src, start_pred):
+    """Lines of the braced blocks that open on a line satisfying start_pred (the opening line included)."""
+    out = set()
+    for i, l in enumerate(src, 1):
+        if start_pred(l):
+            depth, j = 0, i
+            while j <= len(src):
+                depth += src[j - 1].count('{') - src[j - 1].count('}')
+                out.add(j)
+                if depth <= 0 and j > i:
+                    break
+                j += 1
+    return out
+
+
+def fft_kernel_stats(text, kernel):
+    """Per-phase counts of the FP64 FFT kernel (blind_rotate_fft_kernel, fft_kernels.cuh): the phases are the br_fft.cuh
+    calls of br_fft_step.  Per thread and step: fwd2 / fwd3 / inv3 / inv2 run two sweeps, the MAC 512 / THREADS points,
+    and the digit loop of fwd1 and the limb loop of inv1 (br_fft.cuh) two iterations.  Shared-memory and L1 wavefronts
+    are modelled per warp-instruction: a 16 B access per lane is 4 wavefronts, 8 B is 2, 4 B is 1; the tw2 reads of
+    passes 2 / 3 touch 8 distinct entries per warp, 1 wavefront."""
+    kpath = os.path.join(ROOT, 'nufhe_b200', 'csrc', 'fft_kernels.cuh')
+    fpath = os.path.join(ROOT, 'nufhe_b200', 'csrc', 'br_fft.cuh')
+    ksrc = open(kpath).read().splitlines()
+    fsrc = open(fpath).read().splitlines()
+    phase_lines, in_step = {}, False
+    names = {'fft_step_fwd1': 'fwd1', 'fft_fwd2': 'fwd2', 'fft_fwd3': 'fwd3', 'fft_step_mac': 'mac',
+             'fft_inv3': 'inv3', 'fft_inv2': 'inv2', 'fft_step_inv1': 'inv1'}
+    for i, line in enumerate(ksrc, 1):
+        if 'void br_fft_step' in line:
+            in_step = True
+        elif in_step:
+            m = re.search(r'\b(fft_[a-z0-9_]+)(?:<[a-z]+>)?\(', line)
+            if m and m.group(1) in names:
+                phase_lines[i] = names[m.group(1)]
+            if line.startswith('}'):
+                in_step = False
+    twice = block_lines(fsrc, lambda l: 'for (int j = 0; j < 2; j++)' in l or 'for (int limb = 0; limb < 2; limb++)' in l)
+    tw2_lines = {i for i, l in enumerate(fsrc, 1) if 'tw2[' in l}
+    ct = int(re.search(r'BrFftCfgILi(\d+)E', kernel).group(1)) if re.search(r'BrFftCfgILi(\d+)E', kernel) else 2
+    mult = {'fwd1': 1, 'fwd2': 2, 'fwd3': 2, 'mac': 512 // (128 * ct), 'inv3': 2, 'inv2': 2, 'inv1': 1}
+    rx_line = re.compile(r'//## File "([^"]+)", line (\d+)')
+    rx_ins = re.compile(r'^\s+/\*[0-9a-f]+\*/\s+(?:@!?U?P\d+\s+)?([A-Z0-9_.]+)(.*)')
+    cols = ('fp64', 'alu', 'fma', 'lds', 'sts', 'ldg', 'other_lsu', 'uni', 'other', 'total', 'wavefronts')
+    counts = {ph: collections.Counter() for ph in FFT_PHASES}
+    in_kernel, chain, chain_done = False, [], False
+    for ln in text:
+        if ln.startswith('.text.'):
+            in_kernel = kernel in ln
+            chain = []
+            continue
+        if not in_kernel:
+            continue
+        m = rx_line.search(ln)
+        if m:
+            if not chain or chain_done:
+                chain, chain_done = [], False
+            chain.append((m.group(1), int(m.group(2))))
+            continue
+        m = rx_ins.match(ln)
+        if not m:
+            continue
+        chain_done = True
+        phase = next((phase_lines[line] for path, line in chain if path.endswith('fft_kernels.cuh') and line in phase_lines), None)
+        if phase is None:
+            continue
+        w = mult[phase] * (2 if any(path.endswith('br_fft.cuh') and line in twice for path, line in chain) else 1)
+        op = m.group(1)
+        base = op.split('.')[0]
+        c = counts[phase]
+        c['total'] += w
+        if base in FP64:
+            c['fp64'] += w
+        elif base in ('LDS', 'STS', 'LDG'):
+            c[base.lower()] += w
+            width = 16 if '.128' in op else 8 if '.64' in op else 4
+            wf = width // 4 if width > 4 else 1
+            if base == 'LDS' and any(path.endswith('br_fft.cuh') and line in tw2_lines for path, line in chain):
+                wf = 1
+            c['wavefronts'] += w * wf
+        elif pipe_of(op) == 'lsu':
+            c['other_lsu'] += w
+        else:
+            c[pipe_of(op)] += w
+    tot = collections.Counter()
+    for c in counts.values():
+        tot.update(c)
+    return {'kernel': kernel, 'ct_per_cta': ct, 'columns': cols,
+            'phases_per_thread_step': {ph: {k: counts[ph][k] for k in cols} for ph in FFT_PHASES},
+            'per_thread_step': {'fp64': tot['fp64'], 'alu': tot['alu'], 'fma': tot['fma'],
+                                'lsu': tot['lds'] + tot['sts'] + tot['ldg'] + tot['other_lsu'], 'uni': tot['uni'],
+                                'other': tot['other']},
+            'per_thread_step_total': tot['total'],
+            'shared_l1_wavefronts_per_warp_step': tot['wavefronts'],
+            'phases': {ph: counts[ph]['total'] for ph in FFT_PHASES}}
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--lib', default=os.path.join(ROOT, 'nufhe_b200', 'csrc', 'libnufhe_b200.so'))
@@ -92,6 +199,20 @@ def main():
     cubin = [f for f in os.listdir(tmp) if f.endswith('.cubin')][0]
     text = subprocess.run(['nvdisasm', '--print-line-info-inline', '-c', os.path.join(tmp, cubin)],
                           capture_output=True, text=True).stdout.splitlines()
+
+    if 'fft_kernel' in args.kernel:
+        import json
+        d = fft_kernel_stats(text, args.kernel)
+        if args.json:
+            print(json.dumps(d))
+            return 0
+        cols = d['columns']
+        print('%-22s' % 'phase (per thread-step)' + ''.join('%11s' % c for c in cols))
+        for ph, c in d['phases_per_thread_step'].items():
+            print('%-22s' % ph + ''.join('%11.0f' % c[k] for k in cols))
+        tot = {k: sum(c[k] for c in d['phases_per_thread_step'].values()) for k in cols}
+        print('%-22s' % 'step' + ''.join('%11.0f' % tot[k] for k in cols))
+        return 0
 
     # phase = line of kernels.cuh inside br2_step
     kpath = os.path.join(ROOT, 'nufhe_b200', 'csrc', 'kernels.cuh')
